@@ -35,6 +35,22 @@ def tflop_per_image(H, W, steps, cfg):
     return (steps * (2 if cfg else 1) * g["unet"] + 2 * g["enc"] + g["dec"] + g["emasc"]) / 1000.0
 
 
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much, all files together
+
+
+def dump_outputs(path, arrays):
+    """Writes each array as <path>/<name>.npy in float32.  One that would overflow its share of DUMP_BYTES is replaced by a sample of its
+    flattened elements at fixed, seeded positions (the same from run to run), so that two builds can be compared file for file."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 4096  # room for the .npy header
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.nbytes > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).integers(0, a.size, share // a.itemsize))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def peaks():
     try:
         with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
@@ -185,7 +201,13 @@ def main():
     ap.add_argument("--ddim-steps", type=int, default=50)
     ap.add_argument("--guidance", type=float, default=7.5)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the images the last timed step returned as DIR/images.npy "
+                    "(float32; with --gpus > 1 the gathered uint8 batch as 0..255)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "engine":
+        ap.error("--dump-outputs needs --impl engine: the reference arm times a sample of the work and returns no images")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
@@ -215,10 +237,13 @@ def main():
                    num_inference_steps=args.ddim_steps, guidance_scale=args.guidance, generator=gen, output_type=output_type).images
         return out
 
+    last = {}
+
     def step_resident():
         img = call(resident, "pt_u8" if world > 1 else "pt")
         if world > 1:
             dist.all_gather_into_tensor(gather, img)  # the path's only collective: final image gather over NVLink
+        last["images"] = gather if world > 1 else img
 
     def step_e2e():
         dev_in = {k: v.to(dev, non_blocking=True) for k, v in pinned.items()}  # H2D from pinned host memory
@@ -256,6 +281,8 @@ def main():
     sampler.start()
     ms_step, launches = timed(step_resident, args.warmup, args.steps)
     clocks = sampler.summary()
+    if args.dump_outputs and rank == 0:  # before the e2e pass: it writes into the same gather buffer
+        dump_outputs(args.dump_outputs, {k: v.float().cpu().numpy() for k, v in last.items()})
     ms_e2e, _ = timed(step_e2e, 1, args.steps)
 
     # ---- roofline of the dominant kernel: one instrumented eager UNet forward, every conv/GEMM launch bracketed by CUDA events

@@ -1,9 +1,11 @@
-"""Generates tests/golden/clip_text_small.npz by running the REFERENCE'S OWN /root/reference/src/utils/encode_text_word_embedding.py
+"""Generates tests/golden/clip_text_small.npz by running the REFERENCE'S OWN src/utils/encode_text_word_embedding.py
 (imported unmodified) on oracle/ladi_oracle/clip.py:ClipTextEncoder (which exposes the transformers-4.27 attribute surface that file
 touches; its layer arithmetic is pinned against the installed transformers CLIPTextModel in tests/test_oracle_pins.py), CPU fp32,
-seeded small-config weights.  Run in the build container only (needs /root/reference):
+seeded small-config weights.  Needs a checkout of miccunifi/ladi-vton:
 
-    python tests/golden/make_golden_clip.py
+    python tests/golden/make_golden_clip.py <ladi-vton checkout>
+
+tests/test_oracle_pins.py imports this module for build(); only main() reads the checkout.
 """
 import os
 import sys
@@ -12,7 +14,7 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-for p in (ROOT, os.path.join(ROOT, "oracle"), "/root/reference"):
+for p in (ROOT, os.path.join(ROOT, "oracle")):
     sys.path.insert(0, p)
 
 from ladi_oracle.clip import ClipTextEncoder  # noqa: E402
@@ -35,7 +37,8 @@ def build(seed=1234):
     return enc, ids, we
 
 
-def main():
+def main(reference):
+    sys.path.insert(0, reference)
     from src.utils.encode_text_word_embedding import encode_text_word_embedding  # the reference file, unmodified
     enc, ids, we = build()
     with torch.no_grad():
@@ -46,4 +49,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

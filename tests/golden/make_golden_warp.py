@@ -1,9 +1,11 @@
-"""Generates tests/golden/warp_small.npz by running the REFERENCE'S OWN classes -- /root/reference/src/models/ConvNet_TPS.py and
-src/models/UNet.py (+ unet_parts.py), imported unmodified -- CPU fp32, with the seeded weights of ladi_vton_b200.synthetic.
-warp_state_dict.  The reference forward calls `.cuda()` on a few constants (ConvNet_TPS.py:213-216); on this CPU-only container
-`torch.Tensor.cuda` is patched to a no-op for the duration of the script.  Run in the build container only:
+"""Generates tests/golden/warp_small.npz by running the REFERENCE'S OWN classes -- src/models/ConvNet_TPS.py and
+src/models/UNet.py (+ unet_parts.py) of a miccunifi/ladi-vton checkout, imported unmodified -- CPU fp32, with the seeded weights of
+ladi_vton_b200.synthetic.warp_state_dict.  The reference forward calls `.cuda()` on a few constants (ConvNet_TPS.py:213-216); so that
+the script runs without a GPU, `torch.Tensor.cuda` is patched to a no-op for the duration of the script:
 
-    python tests/golden/make_golden_warp.py
+    python tests/golden/make_golden_warp.py <ladi-vton checkout>
+
+tests/test_oracle_pins.py imports this module for build_weights() / build_inputs(); only main() reads the checkout.
 """
 import os
 import sys
@@ -12,7 +14,7 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-for p in (ROOT, os.path.join(ROOT, "oracle"), "/root/reference"):
+for p in (ROOT, os.path.join(ROOT, "oracle")):
     sys.path.insert(0, p)
 
 
@@ -29,7 +31,8 @@ def build_inputs():
     return (torch.rand((2, 3, 256, 192), generator=g) * 2 - 1, torch.rand((2, 21, 256, 192), generator=g), torch.rand((1, 24, 32, 48), generator=g))
 
 
-def main():
+def main(reference):
+    sys.path.insert(0, reference)
     torch.Tensor.cuda = lambda self, *a, **k: self
     from src.models.ConvNet_TPS import ConvNet_TPS as RefTPS  # reference files, unmodified
     from src.models.UNet import UNetVanilla as RefUNet
@@ -49,4 +52,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1])

@@ -254,14 +254,19 @@ def test_coco_body25_mapping_known_answer():
     assert len(m) == 18 and [m[i] for i in range(18)] == [0, 1, 2, 3, 4, 5, 6, 7, 9, 10, 11, 12, 13, 14, 15, 16, 17, 18]
 
 
-def test_bench_algorithmic_flops_known_answers():
-    """bench.py's per-image algorithmic work = SURVEY.md 8(d) / Appendix C (2 flops per MAC of convs, linears, QK^T, PV only):
-    15.61 / 33.06 / 62.15 / 120.32 TFLOP at 512x384 for (N, CFG) = (20, off), (50, off), (50, on), (100, on); 79.43 / 173.68 / 330.77 / 644.93
-    at 1024x768."""
+def _bench():
     import importlib.util
     spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
+    return bench
+
+
+def test_bench_algorithmic_flops_known_answers():
+    """bench.py's per-image algorithmic work = SURVEY.md 8(d) / Appendix C (2 flops per MAC of convs, linears, QK^T, PV only):
+    15.61 / 33.06 / 62.15 / 120.32 TFLOP at 512x384 for (N, CFG) = (20, off), (50, off), (50, on), (100, on); 79.43 / 173.68 / 330.77 / 644.93
+    at 1024x768."""
+    bench = _bench()
     want = {(512, 384): (15.61, 33.06, 62.15, 120.32), (1024, 768): (79.43, 173.68, 330.77, 644.93)}
     for (h, w), vals in want.items():
         got = (bench.tflop_per_image(h, w, 20, False), bench.tflop_per_image(h, w, 50, False), bench.tflop_per_image(h, w, 50, True),
@@ -269,6 +274,24 @@ def test_bench_algorithmic_flops_known_answers():
         for g, v in zip(got, vals):
             assert abs(g - v) < 0.02, (h, w, got, vals)  # SURVEY rounds to 2 decimals
     assert bench.tflop_per_image(256, 192, 50, True) < bench.tflop_per_image(512, 384, 50, True)  # other sizes: area-scaled estimate
+
+
+def test_bench_dump_outputs_whole_or_seeded_sample(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: one float32 .npy per output, whole while it fits the size limit; past it, the same seeded sample of its
+    elements in every run, and the files stay within the limit."""
+    import numpy as np
+    bench = _bench()
+    x = np.arange(24, dtype=np.float64).reshape(2, 3, 4)
+    bench.dump_outputs(str(tmp_path / "a"), {"images": x})
+    got = np.load(tmp_path / "a" / "images.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, x)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096 + 400)  # room for 100 float32 values
+    big = np.random.default_rng(1).random((50, 60), dtype=np.float32)
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), {"images": big})
+    b, c = np.load(tmp_path / "b" / "images.npy"), np.load(tmp_path / "c" / "images.npy")
+    assert b.shape == (100,) and np.array_equal(b, c) and np.isin(b, big).all()
+    assert os.path.getsize(tmp_path / "b" / "images.npy") <= bench.DUMP_BYTES
 
 
 def test_synthetic_workload_matches_survey_spec():
@@ -295,6 +318,7 @@ def test_launch_counter_only_counts_real_launches():
     n = l.ladi_launch_count()
     assert n >= 0 and l.ladi_launch_count() == n
     before = lib.launches
-    with pytest.raises(RuntimeError, match="ladi_add_bf16 failed"):
-        lib.call("ladi_add_bf16", None, None, None, 0, None)
+    # a count that is not a multiple of 8 is refused before any launch, with or without a device (count 0 is a valid, empty launch)
+    with pytest.raises(RuntimeError, match="ladi_add_bf16 failed .*multiple of 8"):
+        lib.call("ladi_add_bf16", None, None, None, 7, None)
     assert lib.launches == before and l.ladi_launch_count() == n
